@@ -57,7 +57,12 @@ def parse():
     ap.add_argument("--ref-time-box", type=float, default=420.0, help="--impl reference: stop after this many seconds")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the auxiliary paths (VI C4, MCTS C3, one-decision latency)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy "
+                                                          "(GPU arm, rank 0; see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 # ----------------------------------------------------------------------------
@@ -377,10 +382,11 @@ def run_b200(a):
         trees = a.trees
     else:
         # default batch: 128 decisions per SM (more work in flight = better overlap of the trees' phases),
-        # capped so that the tree arena (scene + node record + frontier key per node) takes <= 65 % of the free HBM
+        # capped so that the tree arena (scene + node record + frontier key per node) takes <= 65 % of the HBM;
+        # of the whole HBM, not of what is free at the moment, so that the same arguments give the same inputs
         per_tree = (1 + n_exp * N_ACTIONS) * (STATE_BYTES + NODE_BYTES + 8) + 16 * 1024
-        free, _ = torch.cuda.mem_get_info(dev)
-        trees = min(128 * sms, int(0.65 * free / per_tree))
+        total = torch.cuda.get_device_properties(dev).total_memory
+        trees = min(128 * sms, int(0.65 * total / per_tree))
         trees = max(8 * sms, trees // (8 * sms) * (8 * sms))
 
     eng = OPDEngine(_lib.ENV_HIGHWAY, trees, N_ACTIONS, a.budget, a.gamma, keys_in_smem=bool(a.keys_in_smem),
@@ -432,6 +438,8 @@ def run_b200(a):
     # sanity: the timed work really is the full search
     res = eng.result.cpu().numpy()
     assert (res[:, 0] > n_exp).all() and (res[:, 4] == 0).all()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(eng, res, a.dump_outputs)
     mean_children = float((res[:, 0] - 1).mean() / n_exp)
     # ---- e2e: the host-buffer C ABI (b2_opd_create / b2_opd_plan_host): pinned host scenes -> H2D -> search
     #      -> D2H of plans and per-tree results, synchronous, every step ----
@@ -546,6 +554,47 @@ def run_b200(a):
         emit(out)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_TREES = 32         # seeded sample of the batch whose whole node arrays are written
+DUMP_NODES = 64         # seeded sample of node ids whose scene words are written
+
+
+def dump_outputs(eng, res, directory):
+    """--dump-outputs: what the last timed b2_opd_plan() handed to its caller, one .npy file per array.
+
+    Every tree: `result` [trees, 7] (n_nodes, n_leaves, max_depth, terminal_expansions, error, plan_len, tie_node)
+    and `plan`, the trees' plans (plan_len actions each) one after the other.  A seeded sample of trees
+    (`sample_trees`): their node arrays (n_nodes entries each, one tree after the other), and the scene words
+    `state` [sample, nodes, 136] of a seeded sample of node ids (`sample_nodes`, all below n_expansions + 1, so
+    present in every tree).  Entries past a tree's n_nodes or plan_len are left out: the search does not write
+    them, they hold whatever the buffers held before.  Integer outputs are float32 (exact: all are below 2**24), scene words
+    float64, reward / lower / upper float64 as computed."""
+    import numpy as np
+    import torch
+    n_nodes, plan_len = res[:, 0], res[:, 5]
+    out = {"result": res[:, :7].astype(np.float32)}
+    plan = eng.plan_buf[:, :int(plan_len.max())].cpu().numpy()
+    out["plan"] = plan[np.arange(plan.shape[1])[None, :] < plan_len[:, None]].astype(np.float32)   # row-major
+    rng = np.random.default_rng(0)
+    trees = np.sort(rng.choice(eng.n_trees, size=min(DUMP_TREES, eng.n_trees), replace=False))
+    nodes = np.sort(rng.choice(eng.n_expansions + 1, size=min(DUMP_NODES, eng.n_expansions + 1), replace=False))
+    out["sample_trees"], out["sample_nodes"] = trees.astype(np.float32), nodes.astype(np.float32)
+    rows = torch.from_numpy(trees).to(eng.device)
+    written = np.arange(eng.capacity)[None, :] < n_nodes[trees][:, None]
+    for name in ("parent", "first_child", "depth", "count", "meta", "reward", "lower", "upper"):
+        t = getattr(eng, name)
+        x = t.index_select(0, rows).cpu().numpy()[written]
+        out[name] = x.astype(np.float64 if t.dtype == torch.float64 else np.float32)
+    cols = torch.from_numpy(nodes).to(eng.device)
+    out["state"] = eng.state[rows[:, None], cols[None, :]].cpu().numpy().astype(np.float64)
+    size = sum(x.nbytes for x in out.values())
+    if size > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit (use fewer --trees)" % (size, DUMP_LIMIT_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, x in out.items():
+        np.save(os.path.join(directory, name + ".npy"), x)
 
 
 def other_paths(a, dev, world, rank):

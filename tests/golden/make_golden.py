@@ -2,7 +2,7 @@
 reference (/root/reference) on the oracle env models.
 
 Build-container only (the reference tree does not travel to the GPU box);
-the outputs are committed.  Usage:  python tests/golden/make_golden.py
+the outputs are committed.  Usage:  python tests/golden/make_golden.py [--only-highway-vi | --only-host]
 """
 import copy
 import json
@@ -428,8 +428,34 @@ def highway_vi():
     print("highway VI done:", len(out["cases"]), "cases")
 
 
+FACTORY_CASES = [("rl_agents_b200.agents.tree_search.deterministic.DeterministicPlannerAgent", ref_det.DeterministicPlannerAgent,
+                  {"budget": 75}),
+                 ("rl_agents_b200.agents.tree_search.mcts.MCTSAgent", ref_mcts.MCTSAgent, {"budget": 400, "gamma": 0.9})]
+
+
+def host():
+    """The agent shell: the completed configs of the reference agents that the drop-ins replace (built on the
+    large/env_1 finite MDP), and the reference's AbstractTreeSearchAgent driven by the scripted planner of
+    tests/util.py::receding_horizon_schedule -> tests/golden/golden_host.json."""
+    from tests.util import load_mdps, receding_horizon_schedule
+    m = load_mdps()
+    env = envs.FiniteMDPLite(m["large1_T"], m["large1_R"], m["large1_term"])
+    out = {"factory": [{"class": path, "config_in": cfg, "config": dict(ref_cls(env, dict(cfg)).config)}
+                       for path, ref_cls, cfg in FACTORY_CASES],
+           "receding_horizon": {}}
+    for h in (1, 2, 3, 5):
+        plans, log, config = receding_horizon_schedule(ref_abs.AbstractTreeSearchAgent, h)
+        out["receding_horizon"][str(h)] = {"plans": plans, "log": log, "config": config}
+    with open(os.path.join(HERE, "golden_host.json"), "w") as f:
+        json.dump(out, f)
+    print("host done")
+
+
 if __name__ == "__main__":
     if "--only-highway-vi" in sys.argv:
         highway_vi()
+    elif "--only-host" in sys.argv:
+        host()
     else:
         main()
+        host()

@@ -1,16 +1,19 @@
 """CPU tests: the C ABI library exports what include/b2_planner.h declares, the
 spec constants in the CUDA header equal the oracle's fp32 values, and the host
 side of the plugin surface (config merge, defaults, allocation, env hand-off,
-the reference's own agent_factory) behaves like the reference's."""
+construction from a `__class__` string) behaves like the reference's."""
+import importlib
 import os
 import re
+import sys
+import types
+from abc import ABC
 
 import numpy as np
 import pytest
 
 from oracle import envs as oenvs
-from oracle import ref_loader
-from tests.util import load_golden, load_mdps
+from tests.util import load_golden, load_mdps, receding_horizon_schedule
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 M = load_mdps()
@@ -88,22 +91,22 @@ def test_agent_defaults_match_reference_defaults():
         MCTSAgent(env, {"rollout_policy": {"type": "nope"}})
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
-def test_reference_defaults_and_factory_accept_the_drop_in():
-    """The reference's own loader (factory.py:12-27) builds our agents from a
-    `__class__` string, and their completed configs equal the reference agents'."""
-    ref_loader.load_reference()
-    from rl_agents.agents.common.abstract import AbstractAgent as RefAbstractAgent
-    from rl_agents.agents.common.factory import agent_factory
-    from rl_agents.agents.tree_search.deterministic import DeterministicPlannerAgent as RefOPD
-    from rl_agents.agents.tree_search.mcts import MCTSAgent as RefMCTS
+def test_reference_defaults_and_factory_accept_the_drop_in(monkeypatch):
+    """Our agents, built from a `__class__` string the way the reference's loader does it (factory.py:12-27: import
+    the module, take the class, call it with (env, config)), complete their configs to what the reference agents
+    complete them to (tests/golden/golden_host.json), and register as virtual subclasses of the reference's
+    AbstractAgent (an ABC) when that package is loaded in the process."""
+    class RefAbstractAgent(ABC):
+        pass
+    ref_abstract = types.ModuleType("rl_agents.agents.common.abstract")
+    ref_abstract.AbstractAgent = RefAbstractAgent
+    monkeypatch.setitem(sys.modules, "rl_agents.agents.common.abstract", ref_abstract)
     env = oenvs.FiniteMDPLite(M["large1_T"], M["large1_R"], M["large1_term"])
-    for path, ref_cls, cfg in [
-            ("rl_agents_b200.agents.tree_search.deterministic.DeterministicPlannerAgent", RefOPD, {"budget": 75}),
-            ("rl_agents_b200.agents.tree_search.mcts.MCTSAgent", RefMCTS, {"budget": 400, "gamma": 0.9})]:
-        mine = agent_factory(env, dict(cfg, __class__="<class '%s'>" % path))
-        ref = ref_cls(env, dict(cfg))
-        theirs = dict(ref.config)
+    for case in load_golden("golden_host.json")["factory"]:
+        cfg = dict(case["config_in"], __class__="<class '%s'>" % case["class"])
+        module, name = re.fullmatch(r"<class '(.+)\.(\w+)'>", cfg["__class__"]).groups()
+        mine = getattr(importlib.import_module(module), name)(env, cfg)
+        theirs = case["config"]
         ours = {k: v for k, v in mine.config.items() if k != "__class__"}
         assert ours == theirs
         assert isinstance(mine, RefAbstractAgent)
@@ -142,53 +145,16 @@ def test_finite_env_steps_like_the_oracle_env():
         assert a.step(act) == b.step(act)
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("receding_horizon", [1, 2, 3, 5])
 def test_receding_horizon_schedule_matches_the_reference_agent(receding_horizon):
     """The agent shell (own implementation) against the reference's AbstractTreeSearchAgent driven by the
-    same scripted planner: identical plan() outputs, planner calls and step_tree arguments."""
-    ref_loader.load_reference()
-    from rl_agents.agents.tree_search.abstract import AbstractTreeSearchAgent as RefAgent
-    from rl_agents_b200.agents.tree_search.abstract import AbstractTreeSearchAgent as OurAgent
-
-    lengths = [4, 1, 3, 2, 6, 1, 1, 5, 3]
-
-    class Scripted(object):
-        def __init__(self, env, config):
-            self.log, self.k = [], 0
-
-        def plan(self, state, observation):
-            n = lengths[self.k % len(lengths)]
-            self.k += 1
-            self.log.append(("plan", observation))
-            return [10 * self.k + i for i in range(n)]
-
-        def step_tree(self, actions):
-            self.log.append(("step", list(actions)))
-
-        def step_by_reset(self):
-            self.log.append(("reset",))
-
-        def seed(self, seed=None):
-            return [seed]
-
-    class Env(object):
-        unwrapped = property(lambda self: self)
-
-    def run(cls):
-        class A(cls):
-            PLANNER_TYPE = Scripted
-        a = A(Env(), {"receding_horizon": receding_horizon})
-        outs = []
-        for t in range(25):
-            if t == 13:
-                a.reset()
-            outs.append(list(a.plan(t)))
-        return outs, a.planner.log, a.config
-
-    ours, ref = run(OurAgent), run(RefAgent)
-    assert ours[0] == ref[0] and ours[1] == ref[1]
-    assert ours[2] == ref[2]
+    same scripted planner (tests/golden/golden_host.json): identical plan() outputs, planner calls and
+    step_tree arguments."""
+    from rl_agents_b200.agents.tree_search.abstract import AbstractTreeSearchAgent
+    ours = receding_horizon_schedule(AbstractTreeSearchAgent, receding_horizon)
+    ref = load_golden("golden_host.json")["receding_horizon"][str(receding_horizon)]
+    assert ours[0] == ref["plans"] and ours[1] == ref["log"]
+    assert ours[2] == ref["config"]
 
 
 def test_preprocess_env_applies_methods_in_sequence():

@@ -70,6 +70,45 @@ def canonical_tree(first_child, n_children, fields):
     return [[int(n_children[i])] + [f[i] for f in fields] for i in order]
 
 
+def receding_horizon_schedule(agent_cls, receding_horizon):
+    """Drive a subclass of `agent_cls` (an AbstractTreeSearchAgent) by a scripted planner whose plans have fixed
+    lengths, for 25 decisions with a reset() before the 14th: (plan() outputs, the planner's call log, the config).
+    Lists only, so that the result compares equal to its JSON form in tests/golden/golden_host.json."""
+    lengths = [4, 1, 3, 2, 6, 1, 1, 5, 3]
+
+    class Scripted(object):
+        def __init__(self, env, config):
+            self.log, self.k = [], 0
+
+        def plan(self, state, observation):
+            n = lengths[self.k % len(lengths)]
+            self.k += 1
+            self.log.append(["plan", observation])
+            return [10 * self.k + i for i in range(n)]
+
+        def step_tree(self, actions):
+            self.log.append(["step", list(actions)])
+
+        def step_by_reset(self):
+            self.log.append(["reset"])
+
+        def seed(self, seed=None):
+            return [seed]
+
+    class Env(object):
+        unwrapped = property(lambda self: self)
+
+    class A(agent_cls):
+        PLANNER_TYPE = Scripted
+    a = A(Env(), {"receding_horizon": receding_horizon})
+    outs = []
+    for t in range(25):
+        if t == 13:
+            a.reset()
+        outs.append(list(a.plan(t)))
+    return outs, a.planner.log, a.config
+
+
 def ttc_edge_scenes():
     """HighwayLite scenes that exercise the corners of the TTC-grid conversion (docs/HIGHWAY_LITE_SPEC.md section 9):
     absent slots, speeds equal to the grid speeds, integer times / zero distances, headings beyond the cosine clamp,
