@@ -147,6 +147,10 @@ class DistributedVI(object):
             b, e = shard_range(S, self.rank, self.world)
             slab = (np.asarray(transition)[b:e], np.asarray(reward)[b:e], np.asarray(terminal)[b:e],
                     None if nxt is None else np.asarray(nxt)[b:e])
+        if S < self.world:
+            # some rank would own an empty slab (null device tables): its first sweep would fail while the other
+            # ranks block in the exchange.  Every rank knows S and world, so every rank raises here.
+            raise ValueError("%d states cannot be split over %d ranks: every rank needs at least one" % (S, self.world))
         self.n_states = S
         self.engine = VIEngine(mode, slab[0], slab[1], slab[2], nxt=slab[3], gamma=gamma, device=device,
                                row_begin=b, row_end=e, n_states=S, rtol=rtol, atol=atol)

@@ -104,6 +104,33 @@ def test_slab_sharded_value_iteration_matches_single_process():
     assert np.array_equal(np.concatenate([np.array(o) for o in out]), q_ref)
 
 
+def _too_few_states_case(rank, world):
+    """n_states < world leaves the last rank an empty slab: every rank must raise before any allocation or
+    collective, for both exchanges and for full or rank-local tables."""
+    from oracle import envs as oenvs
+    from rl_agents_b200.distributed import DistributedVI
+    P, N, R = oenvs.garnet(1, 2, 2, seed=0)
+    term = np.zeros(1, bool)
+    b, e = shard_range(1, rank, world)
+    out = []
+    for exchange in ("nccl", "p2p"):
+        for local in (False, True):
+            tables = (P[b:e], R[b:e], term[b:e], N[b:e]) if local else (P, R, term, N)
+            try:
+                DistributedVI("sparse", *tables[:3], nxt=tables[3], gamma=0.9, device="cpu", exchange=exchange,
+                              tables_are_local=local, n_states=1 if local else None)
+                out.append(None)
+            except ValueError as err:
+                out.append(str(err))
+    return out
+
+
+def test_distributed_vi_rejects_fewer_states_than_ranks():
+    out = run_world(_too_few_states_case)
+    for msgs in out:
+        assert len(msgs) == 4 and all(m is not None and "1 states cannot be split over 2 ranks" in m for m in msgs), msgs
+
+
 def _merge_case(rank, world):
     from rl_agents_b200.distributed import merge_root_statistics
     counts = torch.tensor([[10, 0, 5], [2, 0, 13]][rank], dtype=torch.int32)

@@ -268,6 +268,97 @@ def test_vi_slabs_compose():
     assert np.array_equal(q, q_full.cpu().numpy())
 
 
+# ------------------------------------------------------------ robust VI ----
+def robust_models_random(mode, M, S, A, seed, shared_rows=0):
+    """M seeded models: int successors [M, S, A] or dense rows [M, S, A, S], rewards [M, S, A].  The first
+    `shared_rows` states of model 1 copy model 0, so both models give equal Q there."""
+    rng = np.random.default_rng(seed)
+    R = rng.uniform(size=(M, S, A))
+    if mode == "deterministic":
+        T = rng.integers(0, S, size=(M, S, A))
+    else:
+        T = rng.uniform(size=(M, S, A, S))
+        T /= T.sum(axis=-1, keepdims=True)
+    T[1:2, :shared_rows] = T[0, :shared_rows]
+    R[1:2, :shared_rows] = R[0, :shared_rows]
+    return T, R
+
+
+def check_robust_vs_numpy(mode, T, R, gamma, iterations):
+    from rl_agents_b200.engine.vi import RobustVIEngine
+    q_ref, sweeps_ref = planners.robust_value_iteration(mode, T, R, gamma, iterations)
+    q, sweeps = RobustVIEngine(mode, T, R, gamma=gamma).solve(iterations)
+    assert sweeps == sweeps_ref
+    assert np.array_equal(q.cpu().numpy(), q_ref)
+    return sweeps
+
+
+# gamma 0.5 converges (allclose) well before 200 sweeps; 0.95 never within 25
+ROBUST_GAMMAS = [(0.5, 200), (0.95, 25)]
+
+
+@pytest.mark.parametrize("gamma,iterations", ROBUST_GAMMAS)
+@pytest.mark.parametrize("S", [1, 127, 1000, 5000])
+@pytest.mark.parametrize("A", [1, 3, 5])
+@pytest.mark.parametrize("M", [1, 2, 8])
+def test_robust_vi_deterministic_vs_numpy(M, A, S, gamma, iterations):
+    T, R = robust_models_random("deterministic", M, S, A, seed=1000 * M + 10 * A + S)
+    sweeps = check_robust_vs_numpy("deterministic", T, R, gamma, iterations)
+    assert (sweeps < iterations) == (gamma == 0.5)
+
+
+@pytest.mark.parametrize("gamma,iterations", ROBUST_GAMMAS)
+@pytest.mark.parametrize("S", [7, 128, 129, 300])
+def test_robust_vi_dense_follows_numpy_pairwise_order(S, gamma, iterations):
+    """Dense rows of < 8, exactly one 128-element pairwise block, and rows numpy splits by recursive halving."""
+    T, R = robust_models_random("stochastic", 3, S, 2, seed=S)
+    sweeps = check_robust_vs_numpy("stochastic", T, R, gamma, iterations)
+    assert (sweeps < iterations) == (gamma == 0.5)
+
+
+@pytest.mark.parametrize("mode,S", [("deterministic", 200), ("stochastic", 150)])
+@pytest.mark.parametrize("iterations", [0, 1, 30])
+def test_robust_vi_few_sweeps_and_tied_models(mode, S, iterations):
+    """0 and 1 sweeps, and models that give equal Q on a third of the (s, a) pairs."""
+    T, R = robust_models_random(mode, 3, S, 3, seed=iterations, shared_rows=S // 3)
+    assert check_robust_vs_numpy(mode, T, R, 0.9, iterations) == iterations
+
+
+@pytest.mark.parametrize("mode,S,A", [("deterministic", 1000, 4), ("stochastic", 129, 3)])
+def test_robust_vi_with_one_model_equals_the_plain_sweep(mode, S, A):
+    import torch
+    from rl_agents_b200.engine.vi import RobustVIEngine, VIEngine
+    T, R = robust_models_random(mode, 1, S, A, seed=3)
+    q_robust, sweeps_robust = RobustVIEngine(mode, T, R, gamma=0.9).solve(40)
+    q_plain, sweeps_plain = VIEngine(mode, T[0], R[0], np.zeros(S, bool), gamma=0.9).solve(40)
+    assert sweeps_robust == sweeps_plain
+    assert torch.equal(q_robust, q_plain)
+
+
+def test_robust_vi_rejects_sparse_mode_and_zero_models():
+    import torch
+    from rl_agents_b200 import _lib
+    from rl_agents_b200.engine.vi import RobustVIEngine
+    T, R = robust_models_random("deterministic", 2, 50, 3, seed=0)
+    with pytest.raises(ValueError):
+        RobustVIEngine("sparse", T, R)
+    eng = RobustVIEngine("deterministic", T, R, gamma=0.9)
+    viol = torch.zeros(1, dtype=torch.int32, device="cuda")
+
+    def rejected(problem, n_models, match):
+        rc = eng.lib.b2_vi_robust_sweep(problem, n_models, _lib.ptr(eng.v[0]), _lib.ptr(eng.q[0]), _lib.ptr(eng.q[1]),
+                                        _lib.ptr(eng.v[1]), _lib.ptr(viol), 0, _lib.current_stream())
+        assert rc != 0 and match in eng.lib.b2_last_error().decode()
+
+    sparse = _lib.VIProblem.from_buffer_copy(eng.problem)
+    sparse.mode = _lib.VI_SPARSE
+    rejected(sparse, 2, "deterministic or stochastic mode")
+    rejected(eng.problem, 0, "bad shape")
+    torch.cuda.synchronize()
+    for t in eng.q + eng.v + [viol]:
+        assert not bool(t.any())
+
+
 # ------------------------------------------------------------------ OPD ----
 def run_opd_finite(mdp, budget, gamma, roots, terminal_reward=0.0, keys_in_smem=False):
     import torch
